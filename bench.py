@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- pseudo-label images/s of the IRN hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 --config selects the BASELINE.json configuration (1-based, as BASELINE.json lists them):
   2  batch=64 synthetic 512x512, multi-scale CAM forward (scales 0.5/1.0/1.5/2.0) + merge            (make_cam body)
@@ -14,6 +14,8 @@ N > 1 is launched by torchrun (one rank per GPU); images shard across ranks (ran
 stride partition) with no data-path collective; NCCL only gathers the per-image label maps to the writer rank (rank 0) on
 a side stream, overlapped with the next step.  Rank 0 prints ONE JSON line.  `--impl reference` times the CPU oracle port
 of the reference's own algorithm (dense (hw)^2 transition matrix squared 8 times, really executed) on the host cores.
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's share) as DIR/<name>.npy; the inputs and weights
+are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -52,6 +54,7 @@ def parse():
     ap.add_argument("--list-limit", type=int, default=0, help="--config 4: ids in the list (default 10,582 * N / 8)")
     ap.add_argument("--step-batch", type=int, default=64, help="--config 4: --step_batch of the step entry points")
     ap.add_argument("--num-workers", type=int, default=-1, help="--config 4: DataLoader workers per GPU")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (64 MB at most)")
     a = ap.parse_args()
     if a.batch <= 0:
         a.batch = 32 if a.config == 5 else 64
@@ -167,10 +170,12 @@ def run_reference(a, rank, out_stream):
     parts = {}
     t_all = time.perf_counter()
     for i in range(steps):
-        _, t = oracle_image(i, "dense")
+        lab, t = oracle_image(i, "dense")
         for k, v in t.items():
             parts[k] = parts.get(k, 0.0) + v / steps
     dt = time.perf_counter() - t_all
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"labels": lab[None]})
     val = steps / dt
     sample = "1 image/step, %d of the requested %d steps executed (bounded: ~35 s of CPU per image), no warm-up, nothing extrapolated: PIL 4-scale " \
              "preprocessing + 4-scale CAM (torch CPU fp32) + EdgeDisplacement + dense 256-step walk (16384^2 fp32 transition matrix, all 8 squarings, " \
@@ -203,6 +208,62 @@ def _claim_stdout():
     keep = os.dup(1)
     os.dup2(2, 1)
     return os.fdopen(keep, "w")
+
+
+# ----------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(dirname, arrays):
+    """Write each array as DIR/<name>.npy: int64 / int32 / float64 data as float64, everything else (labels, masks, classes,
+    float32 maps) as float32 -- exact either way.  The files share DUMP_BYTES: the smaller arrays are stored whole first and
+    the rest split what is left equally; an array larger than its share is stored as the sample of its flattened elements at
+    a seeded set of indices, in increasing order: the same indices for the same shape in every run."""
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {k: np.asarray(v.detach().cpu() if hasattr(v, "detach") else v) for k, v in arrays.items()}
+    left, total = DUMP_BYTES - 1024 * len(arrays), 0          # 1 KB per file for the .npy header
+    for i, name in enumerate(sorted(arrays, key=lambda k: arrays[k].size)):
+        a = arrays[name]
+        dt = np.float64 if a.dtype == np.float64 or (a.dtype.kind in "iu" and a.itemsize >= 4) else np.float32
+        n = left // (len(arrays) - i) // np.dtype(dt).itemsize
+        if a.size > n:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))]
+        a = np.ascontiguousarray(a, dtype=dt)
+        np.save(os.path.join(dirname, name + ".npy"), a)
+        left -= a.nbytes
+        total += a.nbytes
+    print("[bench] --dump-outputs: %d arrays, %.1f MB in %s" % (len(arrays), total / 1e6, dirname), file=sys.stderr)
+
+
+def step_outputs(config_id, out):
+    """What a caller of the timed step receives; per-image lists are concatenated along their first axis, with the
+    per-image lengths beside them (-1: no detection dict for that image)."""
+    import torch
+    if config_id == 5:
+        dets = out["detections"]
+        got = [d for d in dets if d is not None]
+        arrays = {"detections_per_image": [len(d["score"]) if d is not None else -1 for d in dets]}
+        if got:
+            for k in ("score", "class", "mask"):
+                arrays["detection_" + k] = np.concatenate([np.asarray(d[k]) for d in got])
+        return arrays
+    arrays = {"keys_per_image": [len(k) for k in out["keys"]], "keys": np.concatenate(out["keys"]), "cams": torch.cat(out["cams"])}
+    if out.get("high_res") is not None:
+        arrays["high_res"] = torch.cat(out["high_res"])
+    for k in ("labels", "edge", "dp"):
+        if k in out:
+            arrays[k] = out[k]
+    return arrays
+
+
+def stored_outputs(root, tag, n_ids, n_sample=16):
+    """--config 4 returns files: the CAM dicts and label maps the pass `tag` wrote, for a seeded sample of the ids."""
+    from PIL import Image
+    pick = np.sort(np.random.default_rng(0).choice(n_ids, min(n_sample, n_ids), replace=False))
+    cams = [np.load(os.path.join(root, "out_%s_cam" % tag, "2007_%06d.npy" % i), allow_pickle=True).item() for i in pick]
+    return {"ids": pick, "keys_per_image": [len(c["keys"]) for c in cams], "keys": np.concatenate([np.asarray(c["keys"]) for c in cams]),
+            "cams": np.concatenate([np.asarray(c["cam"]) for c in cams]), "high_res": np.concatenate([c["high_res"] for c in cams]),
+            "labels": np.stack([np.asarray(Image.open(os.path.join(root, "out_%s_sem" % tag, "2007_%06d.png" % i))) for i in pick])}
 
 
 # ----------------------------------------------------------------------------------------------- torch-eager context arm
@@ -394,6 +455,8 @@ def run_config4(a, rank, world, local, dev, out_stream):
                     "api": "step.make_cam._work + step.make_sem_seg_labels._work (reference entry points), files in / files out"},
             "gpu_launches": launches, "clocks": clocks, "conv_mode": conv_mode_name(L, cam, dev)}
     if rank == 0:
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, stored_outputs(root, "run%d" % (a.steps - 1), n_ids))
         out_stream.write(json.dumps(line) + "\n")
         out_stream.flush()
         shutil.rmtree(root, ignore_errors=True)
@@ -575,6 +638,8 @@ def main():
     step_ms, n_it = ctypes.c_float(), ctypes.c_int()
     have_rw = a.config in (3, 5) and L.irn_rw_last_step_ms(ctypes.byref(step_ms), ctypes.byref(n_it)) == 0
     L.irn_rw_set_timing(0)
+    if a.dump_outputs and rank == 0:             # before any further step reuses the device buffers
+        dump_outputs(a.dump_outputs, step_outputs(a.config, out))
     step(True)                                   # warm the host path (pinned copies)
     finish()
     ms_e2e, wall_e2e, out, _ = timed(a.steps, True)

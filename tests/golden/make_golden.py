@@ -106,6 +106,34 @@ def gen_to_affinity(ref_indexing):
     np.savez_compressed(os.path.join(HERE, "to_affinity.npz"), **out)
 
 
+def gen_reference_live(ref_indexing):
+    """A second, independent record of the reference's outputs on a few of the inputs above (PathIndex, edge_to_affinity,
+    one random walk, to_affinity forward and gradient), computed afresh rather than read back from the fixtures:
+    tests/test_reference_live.py holds the fixtures to it."""
+    from net import resnet50_irn as ref_irn
+    out = {"path_sha": sha_path_index(ref_indexing.PathIndex(5, (21, 26)))}
+    h, w, r = 12, 17, 5
+    pi = ref_indexing.PathIndex(r, (h + r, w + 2 * r))
+    ep = torch.nn.functional.pad(torch.from_numpy(synth.edge_map(h, w, "uniform", 7)), (r, r, 0, r), value=1.0)
+    out["aff_sha"] = hashlib.sha256(np.ascontiguousarray(ref_indexing.edge_to_affinity(ep[None], pi.path_indices).numpy()).tobytes()).hexdigest()
+    name, hh, ww, C, et, kind, seed = RW_CASES[1]
+    with torch.no_grad():
+        rw = ref_indexing.propagate_to_edge(torch.from_numpy(synth.seeds(C, hh, ww, seed)), torch.from_numpy(synth.edge_map(hh, ww, kind, seed)),
+                                            radius=5, beta=10, exp_times=et)
+    out["rw_name"], out["rw"] = name, rw.numpy().astype(np.float32)
+    r, h, w, B, kind, seed = 5, 24, 31, 3, "uniform", 5          # case "r5" of gen_to_affinity
+    pi = ref_indexing.PathIndex(r, (h, w))
+    stub = types.SimpleNamespace(n_path_lengths=len(pi.path_indices),
+                                 _buffers={ref_irn.AffinityDisplacementLoss.path_indices_prefix + str(i): torch.from_numpy(p) for i, p in enumerate(pi.path_indices)})
+    e = torch.from_numpy(np.stack([synth.edge_map(h, w, kind, seed + b) for b in range(B)])).requires_grad_(True)
+    aff = ref_irn.AffinityDisplacementLoss.to_affinity(stub, e)
+    aff.backward(torch.from_numpy(np.random.RandomState(seed).standard_normal(tuple(aff.shape)).astype(np.float32)))
+    out["toaff_sha"] = hashlib.sha256(np.ascontiguousarray(aff.detach().numpy()).tobytes()).hexdigest()
+    out["toaff_grad"] = e.grad.numpy()
+    np.savez_compressed(os.path.join(HERE, "reference_live.npz"), **out)
+    print("reference_live", {k: getattr(v, "shape", v) for k, v in out.items()})
+
+
 def gen_nets():
     import net.resnet50_cam as rcam
     import net.resnet50_irn as rirn
@@ -362,6 +390,8 @@ def main():
             gen_rw(ref_indexing, c)
     if a.big:
         gen_rw(ref_indexing, RW_BIG)
+    if want("live"):
+        gen_reference_live(ref_indexing)
     if want("inst"):
         gen_instance_fns()
     if want("nets") or want("steps"):
